@@ -238,9 +238,8 @@ class CpuArm:
 
 
 def run_reference_arm(args) -> None:
-    """The reference's own CPU implementation of the path (oracle port: the Rust crate cannot be built in this
-    image), all host threads, same config/metric.  One step = a bounded sample (REF_FRAMES frames) of the batch;
-    the timed region lasts >= 2 s whatever --steps says (steps are repeated until it does)."""
+    """The reference's own CPU implementation of the path (the oracle's C++ port of the Rust crate), all host
+    threads, same config/metric.  One step = a bounded sample (4 frames) of the batch; --steps steps are timed."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -253,23 +252,18 @@ def run_reference_arm(args) -> None:
 
     for _ in range(max(1, min(args.warmup, 3))):
         step()
-    reps, t0 = 0, time.perf_counter()
-    while True:
-        for _ in range(args.steps):
-            step()
-        reps += 1
-        dt = time.perf_counter() - t0
-        if dt >= 2.0:
-            break
-    nsteps = reps * args.steps
-    val = frames * DW * DH * nsteps / 1e6 / dt
+    t0 = time.perf_counter()
+    for _ in range(args.steps):
+        step()
+    dt = time.perf_counter() - t0
+    val = frames * DW * DH * args.steps / 1e6 / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
-        "warmup": args.warmup, "ms_per_step": dt / nsteps * 1e3, "higher_is_better": True, "scaling": "weak",
+        "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": headline_config(args.gpus),
         "cpu_baseline": {"value": val, "unit": UNIT, "cores": arm.threads, "kind": "port",
-                         "sample": f"{frames} of {BATCH} frames per step; " + arm.describe(frames * nsteps, dt)},
+                         "sample": f"{frames} of {BATCH} frames per step; " + arm.describe(frames * args.steps, dt)},
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     emit(line)
@@ -509,6 +503,24 @@ def op_table(kb, dev, peak_gbs: float, quick: bool, n_gpus: int, rank: int) -> d
     return out
 
 
+DUMP_DRAWS = 1 << 22   # draws of the output sample: ~4.15 M distinct elements, ~50 MB of .npy
+
+
+def dump_outputs(out_dir: str, dst) -> None:
+    """--dump-outputs: a fixed sample of the headline output `dst` ([BATCH, 3, DH, DW] f32).  The element indices come
+    from a seeded generator, so two runs (or two builds) write the same elements and compare value for value:
+    resize_normalize_chw.npy holds the values (f32), resize_normalize_chw_index.npy their flat indices into `dst`
+    (f64, exact for any index below 2^53)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.unique(np.random.default_rng(0).integers(0, dst.numel(), DUMP_DRAWS))
+    vals = dst.reshape(-1)[torch.from_numpy(idx).to(dst.device)].cpu().numpy()
+    np.save(os.path.join(out_dir, "resize_normalize_chw.npy"), vals.astype(np.float32))
+    np.save(os.path.join(out_dir, "resize_normalize_chw_index.npy"), idx.astype(np.float64))
+
+
 def e2e_config3(kb, dev, st, n: int, steps: int, n_gpus: int) -> dict:
     import torch
 
@@ -563,7 +575,11 @@ def main() -> None:
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline sample")
     ap.add_argument("--quick", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="tuning sweeps only: skip the host-buffer (e2e) leg; the line then has e2e = null")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of the output of the last timed step (rank 0) to DIR as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     claim_stdout()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -685,6 +701,8 @@ def main() -> None:
         # halves the download — the larger half of the link traffic
         e2e["config3"] = e2e_config3(kb, dev, st, 16 if args.quick else 64, max(2, min(args.steps, 6)), n_gpus)
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:   # dst still holds the last timed step's result: the e2e leg writes host buffers
+        dump_outputs(args.dump_outputs, dst)
     del src, dst
 
     ops = None

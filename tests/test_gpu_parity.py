@@ -907,3 +907,34 @@ def test_video_encode(kb, oracle, dev, w, h):
     np.testing.assert_array_equal(back.numpy(), np.stack([oracle.rgb_from_nv12(oracle.nv12_from_rgb(src[i]), w, h) for i in range(n)]))
     with pytest.raises(kb.ImageError, match="Invalid image size"):
         kb.imgproc.nv12_from_rgb(img, torch.zeros(7, dtype=torch.uint8, device=dev))
+
+
+def test_bench_dump_outputs_is_the_timed_result(kb, oracle, tmp_path):
+    """bench.py --dump-outputs: the same seeded sample of the headline output for any --steps, at most 64 MB, and the
+    sampled elements of frame 0 equal the oracle's fused resize of frame 0's source."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for steps in (1, 2):
+        out = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", "1", "--no-ops", "--no-cpu",
+                            "--no-e2e", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-4000:]
+        lines = [l for l in r.stdout.splitlines() if l.strip()]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps, r.stdout
+        assert sum(f.stat().st_size for f in out.iterdir()) <= 64 << 20
+        dumps.append((np.load(out / "resize_normalize_chw.npy"), np.load(out / "resize_normalize_chw_index.npy")))
+    (vals, idx), (vals2, idx2) = dumps
+    assert vals.dtype == np.float32 and idx.dtype == np.float64 and vals.shape == idx.shape and vals.size > 4_000_000
+    assert np.array_equal(idx, idx2) and np.array_equal(vals.view(np.uint32), vals2.view(np.uint32))
+    sw, sh, dw, dh = 3840, 2160, 1280, 720
+    p = kb.imgproc.NormalizeParams.from_mean_std(kb.IMAGENET_MEAN, kb.IMAGENET_STD)
+    want = oracle.resize_normalize_u8_to_f32_chw(oracle.pattern_u8(sw * sh * 3, 0x12345678).reshape(sh, sw, 3), dw, dh, p.scale, p.bias).reshape(-1)
+    frame0 = idx < want.size
+    assert frame0.sum() > 10_000
+    assert_f32_equal(vals[frame0], want[idx[frame0].astype(np.int64)], "bench dump, frame 0")
+
